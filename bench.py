@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - headline benchmark of the UniVTG hot path on B200 (contract in the task statement).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload NAME]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload NAME] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one synthetic batch:
   cfg3_train BASELINE.json configs[2]: B=32, L_v=75, L_t=32, d=1024, 4 layers: forward + criterion + backward + grad-clip +
@@ -13,6 +13,7 @@ public plugin API (`model(**inputs)`) with pinned HOST inputs, H2D + D2H inside 
 N>1: one process per GPU (torchrun), each rank runs its own replica on its own batch (the path shards by sample; inference
 needs no collective) -> "scaling": "weak".
 --impl reference: the CPU arm (the oracle port of the reference's fp32 PyTorch path, all host threads), rank 0 only.
+--dump-outputs DIR: after the timed steps, rank 0 writes what the last timed step computed to DIR/<name>.npy (see dump_outputs).
 """
 import argparse
 import json
@@ -502,6 +503,33 @@ def emit_json_line(line):
     print(json.dumps(line), flush=True)
 
 
+DUMP_PARAM_SAMPLE = 1 << 20  # parameters written by --dump-outputs: a fixed, seeded sample of this many elements
+
+
+def dump_outputs(path, model, last, train):
+    """Writes what the last timed step returned, as .npy files (about 22 MB for the default workload): the model outputs of its
+    batch, and for a train step also its five losses, the weighted total and a fixed sample of the updated parameters (state_dict
+    order).  Inputs and random draws are seeded, so two builds run with the same arguments can be compared file by file.  The
+    backward's split-K reductions add in fp32 atomics, so train-mode files of two runs agree to a tolerance, not bit for bit
+    (measured on one B200 at 1000 W, 20 steps after 5 warm-up: parameters within 1.1e-3, outputs within 6.1e-3 absolute)."""
+    import numpy as np
+
+    os.makedirs(path, exist_ok=True)
+    out = last["out"]
+    arrays = {k: out[k] for k in ("pred_logits", "pred_spans", "saliency_scores", "vid_mem_proj", "txt_mem_proj")}
+    if train:
+        arrays.update({k: v for k, v in last["losses"].items()})
+        arrays["loss_total"] = last["total"]
+        flat = torch.nn.utils.parameters_to_vector(model.parameters())
+        g = torch.Generator().manual_seed(0)
+        idx = torch.randint(0, flat.numel(), (min(DUMP_PARAM_SAMPLE, flat.numel()),), generator=g).sort().values
+        arrays["params_sample"] = flat[idx.to(flat.device)]
+        arrays["params_sample_index"] = idx.double()
+    for k, v in arrays.items():
+        v = v.detach().cpu()
+        np.save(os.path.join(path, k + ".npy"), (v if v.dtype == torch.float64 else v.float()).numpy())
+
+
 def main():
     _quiet_stdout()
     ap = argparse.ArgumentParser()
@@ -524,7 +552,12 @@ def main():
                     help="zero the flat gradient buffer in front of the backward instead of on a side stream behind the optimizer step")
     ap.add_argument("--no-extras", action="store_true",
                     help="skip the extra legs of the default line (cfg4_train / cfg5_fwd sub-results, GPU torch-eager baseline)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (float32, sample indices float64; rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    torch.manual_seed(0)  # the dropout / DropPath seeds are drawn from torch's CPU generator
     args.warmup = max(args.warmup, 3)
     wl = WORKLOADS[args.workload]
     cfg = synth.CONFIGS[wl["cfg"]]
@@ -599,20 +632,25 @@ def main():
             dist.barrier()
             torch.cuda.synchronize()
 
-    def train_step(inputs, targets):
+    def train_step(inputs, targets, keep=None):
         out = model(**inputs)
         ld = crit(out, targets)
         total = crit.weighted_total(ld)  # = sum(ld[k] * weight_dict[k]) of the reference loop, as one dot product
         opt.zero_grad(set_to_none=True)
         total.backward()
         opt.step()  # clip_grad_norm_(0.1) (reference --grad_clip 0.1) + AdamW
+        if keep is not None:
+            keep.update(out=out, losses=ld, total=total)
         return total
 
-    def device_step(i):
+    def device_step(i, keep=None):
         if train:
-            return train_step(dev_batches[i % n_rot], dev_targets[i % n_rot])
+            return train_step(dev_batches[i % n_rot], dev_targets[i % n_rot], keep)
         with torch.no_grad():
-            return model(**dev_batches[i % n_rot])
+            out = model(**dev_batches[i % n_rot])
+        if keep is not None:
+            keep["out"] = out
+        return out
 
     # ------------------------------------------------ device-resident timing ------------------------------------------------
     for i in range(args.warmup):
@@ -623,14 +661,18 @@ def main():
         sampler.start()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     sync_all()
+    last = {} if args.dump_outputs else None  # what each timed step returned; the last one is written out below
     launches0 = int(lib.univtg_launch_count())
     e0.record()
     for i in range(args.steps):
-        device_step(i)
+        device_step(i, last)
     e1.record()
     sync_all()
     ms_total = e0.elapsed_time(e1)
     gpu_launches = int(lib.univtg_launch_count()) - launches0  # kernels of THIS library launched inside the timed region
+    if last is not None and rank == 0:
+        dump_outputs(args.dump_outputs, model, last, train)
+    last = None
     # host side of the same loop: how long the CPU needs to ENQUEUE a step (5 steps = ~600 launches stay below the driver's launch
     # queue depth, so the host is not throttled by the GPU here).  enqueue time ~ ms_per_step means the step is host-bound.
     sync_all()

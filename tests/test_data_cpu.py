@@ -1,13 +1,11 @@
 """Packed feature shards + batch loader (SURVEY.md section 8 row f-2) against the reference's own loading / collate code
 (main/dataset.py:644-696 feature loading, :534-540 TEF, utils/tensor_utils.py:6-53 pad_sequences_1d), on the CPU."""
 import os
-import sys
 
 import numpy as np
-import pytest
 import torch
 
-from tests.conftest import REFERENCE, has_reference
+from tests.helpers import GOLDEN
 from univtg_b200 import data as D
 
 
@@ -62,32 +60,21 @@ def test_shard_roundtrip_and_loader_batches(tmp_path):
     assert sorted(seen) == list(range(len(anns)))
 
 
-@pytest.mark.skipif(not has_reference(), reason="/root/reference not present on this box")
 def test_prepared_features_and_collate_match_the_reference_code(tmp_path):
-    """prepare_video / prepare_query / the loader's padding against the reference's functions, executed."""
-    if REFERENCE not in sys.path:
-        sys.path.insert(0, REFERENCE)
-    from utils.basic_utils import l2_normalize_np_array
-    from utils.tensor_utils import pad_sequences_1d
-
+    """prepare_video / prepare_query / the loader's padding against what the reference's functions made of the same corpus:
+    main/dataset.py:674-690 + 534-540 with utils.basic_utils.l2_normalize_np_array, then utils.tensor_utils.pad_sequences_1d
+    (tests/golden/reference_pins.npz, written by tests/golden/make_reference_pins.py)."""
+    z = np.load(os.path.join(GOLDEN, "reference_pins.npz"))
+    pad_v, mask_v = torch.from_numpy(z["collate/vid"]), torch.from_numpy(z["collate/vid_mask"])
+    pad_q, mask_q = torch.from_numpy(z["collate/txt"]), torch.from_numpy(z["collate/txt_mask"])
     v_dirs, q_dir, anns = _fake_corpus(tmp_path, seed=5)
-    ref_v, ref_q = [], []
-    for ann in anns[:6]:
-        # main/dataset.py:674-690 + 534-540, re-executed with the reference's helpers
-        fl = [l2_normalize_np_array(np.load(os.path.join(d, f"{ann['vid']}.npz"))["features"].astype(np.float32)) for d in v_dirs]
-        n = min(len(e) for e in fl)
-        v = torch.from_numpy(np.concatenate([e[:n] for e in fl], axis=1))
-        st = torch.arange(0, n, 1.0) / n
-        v = torch.cat([v, torch.stack([st, st + 1.0 / n], dim=1)], dim=1)
-        q = torch.from_numpy(l2_normalize_np_array(np.load(os.path.join(q_dir, f"{ann['qid']}.npz"))["last_hidden_state"].astype(np.float32)))
-        ref_v.append(v)
-        ref_q.append(q)
+    for b, ann in enumerate(anns[:6]):
+        v = pad_v[b, :int(mask_v[b].sum())]
+        q = pad_q[b, :int(mask_q[b].sum())]
         feats = [np.load(os.path.join(d, f"{ann['vid']}.npz"))["features"] for d in v_dirs]
         np.testing.assert_allclose(D.prepare_video(feats), v.numpy(), rtol=1e-6, atol=1e-7)
         np.testing.assert_allclose(D.prepare_query(np.load(os.path.join(q_dir, f"{ann['qid']}.npz"))["last_hidden_state"]), q.numpy(),
                                    rtol=1e-6, atol=1e-7)
-    pad_v, mask_v = pad_sequences_1d(ref_v, dtype=torch.float32, fixed_length=None)
-    pad_q, mask_q = pad_sequences_1d(ref_q, dtype=torch.float32, fixed_length=None)
     path = str(tmp_path / "six.uvshard")
     D.pack_from_npz_dirs(path, anns[:6], v_dirs, q_dir)
     (batch, idx), = list(D.ShardLoader(path, batch_size=6))

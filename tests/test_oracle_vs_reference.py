@@ -1,23 +1,40 @@
-"""Pin the oracle against the LIVE reference (only where /root/reference exists, i.e. the build container)."""
+"""Pin the oracle against the reference: tests/golden/reference_pins.{npz,json} hold what the unmodified reference computes for
+each case below (written by tests/golden/make_reference_pins.py); inputs, weights and random draws are regenerated from seeds."""
+import importlib
+import json
+import os
 import sys
 
+import numpy as np
 import pytest
 import torch
 
-from tests.conftest import REFERENCE, has_reference
+from tests.helpers import GOLDEN
 from univtg_b200 import synth
 
-pytestmark = pytest.mark.skipif(not has_reference(), reason="/root/reference not present on this box")
+OUT_KEYS = ("pred_logits", "pred_spans", "saliency_scores", "vid_mem_proj", "txt_mem_proj")
 
 
-def _ref_model(cfg, sd, **over):
-    if REFERENCE not in sys.path:
-        sys.path.insert(0, REFERENCE)
-    from model.univtg import build_model  # the unmodified reference
+def _pins():
+    with open(os.path.join(GOLDEN, "reference_pins.json")) as f:
+        return json.load(f)
 
-    model, crit = build_model(synth.reference_args(cfg, **over))
-    model.load_state_dict(sd, strict=True)
-    return model, crit
+
+def _ref_out(prefix, keys=OUT_KEYS):
+    z = np.load(os.path.join(GOLDEN, "reference_pins.npz"))
+    return {k: torch.from_numpy(z[f"{prefix}/{k}"]) for k in keys}
+
+
+def _stored(out):
+    """The oracle's outputs as the fixture stores them (vid_mem_proj at every vid_stride-th clip)."""
+    stride = int(np.load(os.path.join(GOLDEN, "reference_pins.npz"))["meta/vid_stride"])
+    return {k: (v[:, ::stride] if k == "vid_mem_proj" else v) for k, v in out.items()}
+
+
+def _assert_losses(loss, ref_loss):
+    assert sorted(loss) == sorted(ref_loss)
+    for k, v in ref_loss.items():
+        assert abs(float(loss[k]) - v) < 5e-6 * max(1.0, abs(v)), k
 
 
 @pytest.mark.parametrize("cfg_name,ragged,batch", [("tiny", True, None), ("tiny", False, 5), ("cfg1", True, 3)])
@@ -26,19 +43,14 @@ def test_forward_and_losses(cfg_name, ragged, batch):
 
     cfg = synth.CONFIGS[cfg_name]
     sd = synth.make_state_dict(cfg, seed=123)
-    model, crit = _ref_model(cfg, sd)
-    model.eval()
     inp = synth.make_inputs(cfg, seed=7, ragged=ragged, batch=batch)
     tgt = synth.make_targets(inp, seed=8)
-    with torch.no_grad():
-        ref = model(**inp)
-        ref_loss = crit(ref, tgt)
+    case = f"{cfg_name}_{int(ragged)}_{batch}"
+    ref = _ref_out("forward/" + case)
     out = O.forward(sd, cfg, **inp)
-    for k in ("pred_logits", "pred_spans", "saliency_scores", "vid_mem_proj", "txt_mem_proj"):
-        torch.testing.assert_close(out[k], ref[k].double(), rtol=2e-5, atol=2e-5)
-    loss = O.criterion(out, tgt)
-    for k, v in ref_loss.items():
-        assert abs(float(loss[k]) - float(v)) < 5e-6 * max(1.0, abs(float(v))), k
+    for k in OUT_KEYS:
+        torch.testing.assert_close(_stored(out)[k], ref[k].double(), rtol=2e-5, atol=2e-5)
+    _assert_losses(O.criterion(out, tgt), _pins()["forward_loss/" + case])
 
 
 def test_bool_masks_of_the_highlight_path_give_the_same_outputs():
@@ -48,14 +60,11 @@ def test_bool_masks_of_the_highlight_path_give_the_same_outputs():
 
     cfg = synth.CONFIGS["tiny"]
     sd = synth.make_state_dict(cfg, seed=11)
-    model, _ = _ref_model(cfg, sd)
-    model.eval()
     inp = synth.make_inputs(cfg, seed=3, ragged=True, batch=4)
     as_bool = dict(inp, src_vid_mask=inp["src_vid_mask"].bool(), src_txt_mask=inp["src_txt_mask"].bool())
-    with torch.no_grad():
-        ref_f, ref_b = model(**inp), model(**as_bool)
-    out = O.forward(sd, cfg, **as_bool)
-    for k in ("pred_logits", "pred_spans", "saliency_scores", "vid_mem_proj", "txt_mem_proj"):
+    ref_f, ref_b = _ref_out("bool_masks/float"), _ref_out("bool_masks/bool")
+    out = _stored(O.forward(sd, cfg, **as_bool))
+    for k in OUT_KEYS:
         torch.testing.assert_close(ref_b[k], ref_f[k], rtol=0, atol=0)
         torch.testing.assert_close(out[k], ref_f[k].double(), rtol=2e-5, atol=2e-5)
 
@@ -67,12 +76,9 @@ def test_droppath_scales_match_reference_train_mode():
 
     cfg = synth.CONFIGS["tiny"]
     sd = synth.make_state_dict(cfg, seed=5)
-    model, _ = _ref_model(cfg, sd, droppath=0.3, input_dropout=0.0)
-    model.train()
     inp = synth.make_inputs(cfg, seed=9, ragged=True, batch=6)
     B = inp["src_vid"].shape[0]
-    torch.manual_seed(77)
-    ref = model(**inp)
+    ref = _ref_out("droppath", ("pred_spans", "pred_logits"))  # reference in train mode, droppath 0.3, after manual_seed(77)
     torch.manual_seed(77)
     keep = 0.7
     scales = torch.stack([torch.floor(keep + torch.rand((B, 1, 1))).flatten() / keep for _ in range(2 * cfg["enc_layers"])])
@@ -82,11 +88,10 @@ def test_droppath_scales_match_reference_train_mode():
 
 
 def test_state_dict_keys_and_shapes_match_reference():
+    pins = _pins()
     for name in ("tiny", "cfg1"):
-        cfg = synth.CONFIGS[name]
-        model, _ = _ref_model(cfg, synth.make_state_dict(cfg))
-        ref = {k: tuple(v.shape) for k, v in model.state_dict().items()}
-        assert list(ref.items()) == list(synth.state_dict_shapes(cfg).items())
+        ref = [(k, tuple(s)) for k, s in pins["state_dict/" + name]]
+        assert ref == list(synth.state_dict_shapes(synth.CONFIGS[name]).items())
 
 
 def test_input_dropout_masks_match_reference_train_mode():
@@ -98,83 +103,41 @@ def test_input_dropout_masks_match_reference_train_mode():
 
     cfg = synth.CONFIGS["tiny"]
     sd = synth.make_state_dict(cfg, seed=5)
-    model, crit = _ref_model(cfg, sd, droppath=0.0, input_dropout=0.5)
-    model.train()
     inp = synth.make_inputs(cfg, seed=9, ragged=True, batch=6)
     tgt = synth.make_targets(inp, seed=10)
     B, Lv, Lt, d = inp["src_vid"].shape[0], inp["src_vid"].shape[1], inp["src_txt"].shape[1], cfg["hidden_dim"]
-    torch.manual_seed(31)
-    ref = model(**inp)
-    ref_loss = crit(ref, tgt)
+    ref = _ref_out("input_dropout", ("pred_logits", "pred_spans", "vid_mem_proj", "txt_mem_proj"))  # after manual_seed(31)
     torch.manual_seed(31)
     shapes = [(B, Lv, cfg["v_feat_dim"]), (B, Lv, d), (B, Lt, cfg["t_feat_dim"]), (B, Lt, d)]
     masks = [torch.nn.functional.dropout(torch.ones(s), 0.5, True) for s in shapes]
     out = O.forward(sd, cfg, **inp, drop_masks=masks)
-    for k in ("pred_logits", "pred_spans", "vid_mem_proj", "txt_mem_proj"):
-        torch.testing.assert_close(out[k], ref[k].detach().double(), rtol=2e-5, atol=2e-5)
-    loss = O.criterion(out, tgt)
-    for k, v in ref_loss.items():
-        assert abs(float(loss[k]) - float(v)) < 5e-6 * max(1.0, abs(float(v))), k
+    for k in ref:
+        torch.testing.assert_close(_stored(out)[k], ref[k].double(), rtol=2e-5, atol=2e-5)
+    _assert_losses(O.criterion(out, tgt), _pins()["input_dropout_loss"])
 
 
 def test_hl_loss_list_matches_reference():
     """dset_type 'hl' / 'vs': losses = ['labels', 'saliency'] and the targets carry no timestamp / span_labels_nn
     (model/univtg.py:438-439, main/dataset.py:1118-1126)."""
     from oracle import univtg_oracle as O
+    from univtg_b200 import build_model
 
     cfg = synth.CONFIGS["tiny"]
     sd = synth.make_state_dict(cfg, seed=5)
-    model, crit = _ref_model(cfg, sd, dset_type="hl")
-    assert crit.losses == ["labels", "saliency"]
-    model.eval()
+    pins = _pins()["hl"]
+    assert pins["criterion_losses"] == ["labels", "saliency"]
+    assert build_model(synth.reference_args(cfg, dset_type="hl"))[1].losses == pins["criterion_losses"]
     inp = synth.make_inputs(cfg, seed=9, ragged=True, batch=6)
     full = synth.make_targets(inp, seed=10)
     tgt = {"saliency_scores": full["saliency_scores"], "saliency_pos_labels": full["saliency_pos_labels"],
            "timestamp_mask": full["timestamp_mask"], "timestamp_window": 1 * (full["saliency_scores"] > 0)}
-    with torch.no_grad():
-        ref = model(**inp)
-        ref_loss = crit(ref, tgt)
-    assert sorted(ref_loss) == ["loss_f", "loss_s_inter", "loss_s_intra"]
+    assert sorted(pins["loss"]) == ["loss_f", "loss_s_inter", "loss_s_intra"]
     loss = O.criterion(O.forward(sd, cfg, **inp), tgt, losses=("labels", "saliency"))
-    assert sorted(loss) == sorted(ref_loss)
-    for k, v in ref_loss.items():
-        assert abs(float(loss[k]) - float(v)) < 5e-6 * max(1.0, abs(float(v))), k
+    _assert_losses(loss, pins["loss"])
 
 
-def _stub_dataset_deps():
-    """main.dataset imports h5py and nncore at module level but the MR evaluation loop never calls into them (SURVEY 8c)."""
-    import types
-
-    if "h5py" not in sys.modules:
-        sys.modules["h5py"] = types.ModuleType("h5py")
-    if "nncore" not in sys.modules:
-        nn_ = types.ModuleType("nncore")
-        ds = types.ModuleType("nncore.dataset")
-
-        class _Registry:
-            def register(self, *a, **k):
-                return lambda c: c
-
-        ds.DATASETS = _Registry()
-        par = types.ModuleType("nncore.parallel")
-        par.DataContainer = object
-        nn_.dataset, nn_.parallel = ds, par
-        sys.modules.update({"nncore": nn_, "nncore.dataset": ds, "nncore.parallel": par})
-    if REFERENCE not in sys.path:
-        sys.path.insert(0, REFERENCE)
-
-
-@pytest.mark.parametrize("sort", [True, False])
-def test_decode_restatement_matches_compute_mr_results(sort):
-    """Pins oracle/postproc_oracle.decode_mr + saliency_lists to the reference's own evaluation loop: compute_mr_results
-    (main/inference_mr.py:86-193) is executed here with a stub model / loader that replay fixed outputs."""
-    from argparse import Namespace
-
-    from oracle import postproc_oracle as PO
-
-    _stub_dataset_deps()
-    import main.inference_mr as M
-
+def decode_case():
+    """Fixed model outputs replayed through the reference's evaluation loop: (outputs, timestamps, video mask, durations, Lt)."""
     g = torch.Generator().manual_seed(1234)
     B, Lv, Lt = 5, 23, 7
     lens = [23, 9, 17, 1, 12]
@@ -188,72 +151,54 @@ def test_decode_restatement_matches_compute_mr_results(sort):
     sal = torch.randn(B, Lv, generator=g)
     ts = ((torch.arange(Lv, dtype=torch.float32) + 0.5) / Lv)[None, :, None].expand(B, Lv, 2).contiguous()
     durs = [150.0, 33.3, 126.0, 2.0, 150.0]
-    outputs = {"pred_logits": pred_logits, "pred_spans": pred_spans, "saliency_scores": sal}
+    return {"pred_logits": pred_logits, "pred_spans": pred_spans, "saliency_scores": sal}, ts, vmask, durs, Lt
 
-    class FakeModel:
-        def eval(self):
-            return self
 
-        def __call__(self, **kw):
-            return {k: v.clone() for k, v in outputs.items()}
+@pytest.mark.parametrize("sort", [True, False])
+def test_decode_restatement_matches_compute_mr_results(sort):
+    """Pins oracle/postproc_oracle.decode_mr + saliency_lists to the reference's own evaluation loop: what compute_mr_results
+    (main/inference_mr.py:86-193) returned with a stub model / loader that replay the outputs of decode_case()."""
+    from oracle import postproc_oracle as PO
 
-    meta = [{"qid": i, "query": "q", "vid": "v", "duration": durs[i]} for i in range(B)]
-    batch = {"query_feat": (torch.zeros(B, Lt, 4), torch.ones(B, Lt)), "video_feat": (torch.zeros(B, Lv, 4), vmask),
-             "timestamp": (ts, vmask), "timestamp_window": (torch.zeros(B, Lv),), "span_labels_nn": (torch.zeros(B, Lv, 2),)}
-    opt = Namespace(device="cpu", pin_memory=False, span_loss_type="l1", model_id="univtg", eval_mode=None,
-                    no_sort_results=not sort, debug=False, round_multiple=0, clip_length=2)
-    res, _ = M.compute_mr_results(FakeModel(), [(meta, batch)], opt)
-    rows = PO.decode_mr(pred_logits, pred_spans, ts, vmask, durs, sort=sort)
-    sal_lists = PO.saliency_lists(sal, vmask)
-    assert len(res) == B
-    for b in range(B):
+    outputs, ts, vmask, durs, _ = decode_case()
+    res = _pins()[f"compute_mr_results/sort={sort}"]
+    rows = PO.decode_mr(outputs["pred_logits"], outputs["pred_spans"], ts, vmask, durs, sort=sort)
+    sal_lists = PO.saliency_lists(outputs["saliency_scores"], vmask)
+    assert len(res) == vmask.shape[0]
+    for b in range(len(res)):
         assert res[b]["pred_relevant_windows"] == rows[b], b
         assert res[b]["pred_saliency_scores"] == sal_lists[b], b
 
 
 def test_reference_setup_model_builds_the_plugin(tmp_path):
     """Boundary (SURVEY 8b): main.config.setup_model does importlib.import_module('model.' + opt.model_id).build_model(opt)
-    (main/config.py:341-342).  With the one-line shim of INTEGRATION.md on sys.path as model/univtg_b200.py the reference's own
-    factory builds (model, criterion, optimizer, lr_scheduler); AdamW sees the same parameter names / order / shapes as for
-    --model_id univtg, and a checkpoint saved from the reference model loads strict=True after `module.` stripping."""
-    import importlib
-
-    _stub_dataset_deps()
-    # the reference's `model` is a namespace package (no __init__.py): a second model/ directory on sys.path joins it, which is
-    # how the one-file shim is tried out without touching /root/reference (a maintainer drops the file into model/ instead)
+    (main/config.py:341-342).  With the one-line shim of INTEGRATION.md on sys.path as model/univtg_b200.py that import builds
+    (model, criterion); AdamW (all parameters with requires_grad, main/config.py:348-349) sees the same parameter names / order /
+    shapes as setup_model gave the reference for --model_id univtg, and a checkpoint in the reference's layout (DDP prefixes every
+    key with 'module.', train_vlp_ddp.py:157-164; setup_model strips it) loads strict=True."""
+    ref = _pins()["setup_model"]
     shim = tmp_path / "model"
     shim.mkdir()
     (shim / "univtg_b200.py").write_text("from univtg_b200.plugin import build_model  # noqa: F401\n")
     sys.path.append(str(tmp_path))
     importlib.invalidate_caches()
     try:
-        cfgmod = importlib.import_module("main.config")
         cfg = synth.CONFIGS["tiny"]
-        class _CpuDevice(str):  # the reference reads opt.device both as torch.device(opt.device) (model/univtg.py:410) and as
-            def __int__(self):  # int(opt.device) >= 0 (main/config.py:344; the CLI passes 0 = cuda, which this box lacks)
-                return -1
-
-        extra = dict(device=_CpuDevice("cpu"), gpu_id=0, lr=1e-4, wd=1e-4, lr_warmup=[10], lr_drop=400, lr_gamma=0.1, resume=None, resume_all=False)
-        built = {}
-        for mid in ("univtg", "univtg_b200"):
-            opt = synth.reference_args(cfg, model_id=mid, **extra)
-            torch.manual_seed(0)
-            built[mid] = cfgmod.setup_model(opt)
-        (m_ref, c_ref, o_ref, s_ref), (m_new, c_new, o_new, s_new) = built["univtg"], built["univtg_b200"]
+        opt = synth.reference_args(cfg, model_id="univtg_b200", gpu_id=0, lr=1e-4, wd=1e-4, lr_warmup=[10], lr_drop=400,
+                                   lr_gamma=0.1, resume=None, resume_all=False)
+        torch.manual_seed(0)
+        m_new, c_new = importlib.import_module("model." + opt.model_id).build_model(opt)
         assert type(m_new).__module__ == "univtg_b200.plugin"
-        assert type(s_new).__name__ == type(s_ref).__name__ == "WarmupStepLR"
-        names_ref = [(n, tuple(p.shape)) for n, p in m_ref.named_parameters() if p.requires_grad]
-        names_new = [(n, tuple(p.shape)) for n, p in m_new.named_parameters() if p.requires_grad]
-        assert names_ref == names_new
-        assert [tuple(p.shape) for p in o_ref.param_groups[0]["params"]] == [tuple(p.shape) for p in o_new.param_groups[0]["params"]]
-        assert c_new.weight_dict == c_ref.weight_dict and c_new.losses == c_ref.losses
-        # checkpoint written by the reference training loop (DDP prefixes every key with 'module.', train_vlp_ddp.py:157-164)
-        ckpt = tmp_path / "ckpt.pt"
-        torch.save({"model": {"module." + k: v for k, v in m_ref.state_dict().items()}, "epoch": 3}, ckpt)
-        opt = synth.reference_args(cfg, model_id="univtg_b200", **dict(extra, resume=str(ckpt)))
-        m_loaded = cfgmod.setup_model(opt)[0]
-        for (k1, v1), (k2, v2) in zip(m_ref.state_dict().items(), m_loaded.state_dict().items()):
-            assert k1 == k2 and torch.equal(v1, v2)
+        params = [(n, list(p.shape)) for n, p in m_new.named_parameters() if p.requires_grad]
+        assert params == [tuple(x) for x in ref["named_parameters"]]
+        assert [s for _, s in params] == ref["optimizer_params"]
+        assert c_new.weight_dict == ref["weight_dict"] and c_new.losses == ref["losses"]
+        g = torch.Generator().manual_seed(3)
+        ckpt = {"module." + k: torch.randn(s, generator=g) for k, s in ref["state_dict"]}
+        m_new.load_state_dict({k.replace("module.", ""): v for k, v in ckpt.items()}, strict=True)
+        for (k1, v1), (k2, v2) in zip(ckpt.items(), m_new.state_dict().items()):
+            assert k1 == "module." + k2 and torch.equal(v1, v2)
     finally:
         sys.path.remove(str(tmp_path))
         sys.modules.pop("model.univtg_b200", None)
+        sys.modules.pop("model", None)

@@ -2,12 +2,10 @@
 import json
 import os
 import random
-import sys
 
 import pytest
 import torch
 
-from tests.conftest import REFERENCE, has_reference
 from tests.helpers import GOLDEN
 
 
@@ -27,23 +25,31 @@ def test_oracle_nms_matches_reference_fixtures():
         assert got == c["expected"], (c["nms_thd"], c["max_after_nms"], len(c["rows"]))
 
 
-@pytest.mark.skipif(not has_reference(), reason="/root/reference not present on this box")
-def test_oracle_nms_matches_live_reference_random():
-    if REFERENCE not in sys.path:
-        sys.path.insert(0, REFERENCE)
-    from utils.temporal_nms import temporal_nms as ref_nms
-
-    from oracle import postproc_oracle as P
-
+def random_nms_cases():
+    """300 seeded (rows, nms_thd, max_after_nms) cases: empty lists, zero-length windows, zero scores."""
     rng = random.Random(3)
+    cases = []
     for _ in range(300):
         n = rng.choice([0, 1, 2, 5, 10, 40])
         rows = []
         for _ in range(n):
             st = round(rng.uniform(0, 100), 4)
             rows.append([st, round(st + rng.choice([0.0, rng.uniform(0, 50)]), 4), round(rng.choice([0.0, rng.random()]), 4)])
-        thd, ma = rng.choice([0.1, 0.5, 0.7, 0.9]), rng.choice([1, 3, 10, 100])
-        assert P.temporal_nms([list(r) for r in rows], thd, ma) == ref_nms([list(r) for r in rows], thd, ma)
+        cases.append((rows, rng.choice([0.1, 0.5, 0.7, 0.9]), rng.choice([1, 3, 10, 100])))
+    return cases
+
+
+def test_oracle_nms_matches_live_reference_random():
+    """Against what the reference's utils.temporal_nms.temporal_nms returned for random_nms_cases()
+    (tests/golden/reference_pins.json, written by tests/golden/make_reference_pins.py)."""
+    from oracle import postproc_oracle as P
+
+    with open(os.path.join(GOLDEN, "reference_pins.json")) as f:
+        expected = json.load(f)["temporal_nms_random"]
+    cases = random_nms_cases()
+    assert len(expected) == len(cases)
+    for (rows, thd, ma), want in zip(cases, expected):
+        assert P.temporal_nms([list(r) for r in rows], thd, ma) == want
 
 
 def _random_batch(B, Lv, seed, ties=True):
